@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark of the B200 path_tracer hot path (BASELINE.json metric: Msamples/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--spp-per-step S]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--spp-per-step S] [--dump-outputs DIR]
 
 Workload (config C1 of BASELINE.json): Cornell box + 868,480-triangle Lambert mesh (procedural stand-in for the
 Stanford dragon, see tungsten_b200/synth.py), 1920x1080, path_tracer, max_bounces 64, Sobol sampler,
@@ -17,6 +17,9 @@ followed by the path's single collective, an all-gather of the tile-major float3
             write, SURVEY 8d) / CUDA-event duration of the launches in the timed region / measured HBM peak.
 `cpu_baseline`: the reference's own CPU renderer (oracle/_ref/tungsten, built from /root/reference by
             oracle/ref/Makefile) on this box's host cores, same scene, bounded sample (fewer spp).
+`--dump-outputs DIR`: after the timed steps, the framebuffer a caller reads back from the last one (running mean and
+            sample count of every pixel, the whole frame gathered on rank 0) as DIR/mean.npy and DIR/count.npy (float32).
+            Scene and seed are fixed, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -33,6 +36,8 @@ sys.path.insert(0, ROOT)
 
 W, H = 1920, 1080
 ALG_BYTES_PER_QUERY = 48
+DUMP_LIMIT_BYTES = 64 << 20         # --dump-outputs: larger frames are written as a fixed, seeded sample of pixels
+DUMP_SAMPLE_PIXELS = 1 << 21
 CONFIGS = {
     "c1": {"res": (1920, 1080), "label": "C1: Cornell box + 868,480-tri Lambert mesh (procedural dragon stand-in), 1920x1080, path_tracer, max_bounces 64, Sobol"},
     "c2": {"res": (1920, 1080), "label": "C2: room with 327,680-triangle furniture stand-ins in rough conductor / rough dielectric / plastic / rough plastic, checker floor, quad + mesh lights + importance-sampled HDR environment, 1920x1080, max_bounces 16, Sobol"},
@@ -227,9 +232,30 @@ STREAM_BYTES = {
 }
 
 
-def _measure(ctx, args, torch, dist, rank, world, local_rank, W, H, seed, steps, warmup, spp_per_step, e2e=True):
+def dump_outputs(out_dir, mean, count):
+    """Writes the framebuffer as DIR/mean.npy (H x W x 3) and DIR/count.npy (H x W), float32.  A frame above
+    DUMP_LIMIT_BYTES is written as the same DUMP_SAMPLE_PIXELS pixels every run (seed 0, ascending row-major index in
+    DIR/pixel_index.npy, float64): mean.npy is then N x 3 and count.npy N."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    h, w = count.shape
+    arrays = {"mean": mean.astype(np.float32), "count": count.astype(np.float32)}
+    if h*w*16 > DUMP_LIMIT_BYTES:
+        idx = np.sort(np.random.default_rng(0).choice(h*w, DUMP_SAMPLE_PIXELS, replace=False))
+        arrays = {"mean": arrays["mean"].reshape(h*w, 3)[idx], "count": arrays["count"].reshape(h*w)[idx],
+                  "pixel_index": idx.astype(np.float64)}
+    else:
+        stale = os.path.join(out_dir, "pixel_index.npy")       # left by an earlier sampled dump into the same DIR
+        if os.path.exists(stale):
+            os.remove(stale)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def _measure(ctx, args, torch, dist, rank, world, local_rank, W, H, seed, steps, warmup, spp_per_step, e2e=True, keep_output=False):
     """Times `steps` steps of the hot path on this rank's tile share (device-resident), then the same through the host-buffer
-    C-ABI call.  Returns a dict of raw numbers (rank-local + reduced)."""
+    C-ABI call.  Returns a dict of raw numbers (rank-local + reduced); with keep_output, also the framebuffer after the
+    timed steps (on rank 0: the whole frame)."""
     import numpy as np
     from tungsten_b200 import integrator
     all_tiles = integrator.dice_tiles(W, H, seed)
@@ -287,6 +313,12 @@ def _measure(ctx, args, torch, dist, rank, world, local_rank, W, H, seed, steps,
     stop.set(); th.join()
     st = ctx.stats()
     out = {"secs": secs, "wall": wall, "clk": clk, "spp_step": spp_step, "n_my_pix": sum(t.w*t.h for t in my_tiles), "st": st}
+    if keep_output:
+        if world > 1:                                 # the last all-gather holds every rank's share of the running mean
+            ctx.clear()
+            for r in range(world):
+                ctx.unpack_tiles(shares[r], recv.data_ptr() + 4*r*max_pix*3, spp_step*steps)
+        out["framebuffer"] = ctx.read_framebuffer()
     coll_ms = sum(a.elapsed_time(b) for a, b in coll_events)
     per_rank = [my_secs*1e3, st.total_ms, st.trace_ms, st.shadow_ms, coll_ms, float(st.samples)]
     if world > 1:
@@ -378,6 +410,8 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-other-configs", action="store_true", help="skip the short C2/C3/C4 measurements added to the C1 line")
     ap.add_argument("--config", default="c1", choices=sorted(CONFIGS))
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the framebuffer the last timed step left as DIR/<name>.npy (float32)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -415,7 +449,10 @@ def main():
     seed = 0xBA5EBA11
     scene_path, ctx, build_times = load(args.config)
     info = ctx.scene_info()
-    m = _measure(ctx, args, torch, dist, rank, world, local_rank, W, H, seed, args.steps, args.warmup, args.spp_per_step)
+    m = _measure(ctx, args, torch, dist, rank, world, local_rank, W, H, seed, args.steps, args.warmup, args.spp_per_step,
+                 keep_output=args.dump_outputs is not None)
+    if args.dump_outputs is not None and rank == 0:
+        dump_outputs(args.dump_outputs, *m["framebuffer"])
     st = m["st"]
     tot_samples, tot_rays, tot_hits, tot_launches = m["tot"]
     value = tot_samples/m["secs"]/1e6

@@ -14,8 +14,11 @@ needs /root/reference and the binaries built by `make -C oracle/ref`).
   <scene>/ref_pathseed.pfm   framebuffer of oracle/_ref/tungsten_pathseed (per-path reseed contract)
   <scene>/ref_stock.pfm      framebuffer of the UNMODIFIED reference binary
   hair_sky/                  curves + hair BCSDF lit by the shipped hair scene's own emitters (infinite_sphere_cap + skydome);
-                             scene_sky.pfm = the image Skydome::prepareForRender computed, dumped through the reference's classes
+                             scene_sky_top.pfm = the image Skydome::prepareForRender computed, dumped through the reference's
+                             classes, down to the horizon (the 2:1 image is zero below it; tests pad it back: "scene_sky.pfm")
   cornell_adaptive/          the same with renderer.adaptive_sampling = true, 48 spp in three 16-spp steps
+  materialtest/, hair_shipped/   shrunk copies of two scenes the reference ships + its renders of them (make_shipped_scenes)
+  sobol_reference.json       checksum and sampled entries of the reference's Sobol direction matrices
 
 The fixtures are small (64x64) so that the CPU test-suite stays fast; they travel to the GPU box with the
 repository, /root/reference does not.
@@ -621,6 +624,7 @@ def make_kat_curves():
 
 
 def make_scenes(only=None):
+    import numpy as np
     from tungsten_b200 import synth
     scenes = {}
     res, spp = (64, 64), 8
@@ -650,7 +654,12 @@ def make_scenes(only=None):
     scenes["dirac"] = synth.dirac_room(os.path.join(HERE, "dirac"), "scene", res=res, spp=spp, subdiv=2)
     # the two emitters of the shipped hair scene: infinite_sphere_cap (sampled sun) + skydome (unsampled sky); min_bounces 1 as shipped
     scenes["hair_sky"] = synth.hair_scene(os.path.join(HERE, "hair_sky"), "scene", n_curves=300, res=res, spp=spp, shipped_lights=True, min_bounces=1)
-    dump_sky_image(scenes["hair_sky"], os.path.join(HERE, "hair_sky", "scene_sky.pfm"))
+    # the sky image is zero below the horizon (its lower 126 rows): only the rows above are stored, tests pad the rest
+    sky = dump_sky_image(scenes["hair_sky"], os.path.join(tempfile.mkdtemp(), "scene_sky.pfm"))
+    from tungsten_b200 import scene as S
+    above = np.where(sky.any(axis=(1, 2)))[0]
+    assert above[0] == 0 and not sky[above[-1] + 1:].any() and 2*len(sky) == sky.shape[1]
+    S.save_pfm(os.path.join(HERE, "hair_sky", "scene_sky_top.pfm"), sky[:above[-1] + 1])
     # adaptive sampling (PathTraceIntegrator::generateWork): three 16-spp steps, the 2nd and 3rd distributed by the blocks' error
     ad = synth.cornell_box(res=res, spp=48)
     ad["renderer"].update(adaptive_sampling=True, spp_step=16)
@@ -668,11 +677,114 @@ def make_scenes(only=None):
         print("golden:", name)
 
 
+def make_sobol_reference():
+    """The direction matrices of the reference's src/thirdparty/sobol/sobol.cpp, as far as the library uses them (first 32
+    of 52 bits, 1024 dimensions): their SHA-256 and 256 entries at seeded positions -> sobol_reference.json."""
+    import hashlib
+    import re
+    import numpy as np
+    txt = open(os.path.join(REF, "src", "thirdparty", "sobol", "sobol.cpp")).read()
+    body = txt[txt.index("matrices[Matrices::num_dimensions"):]
+    nums = np.array([int(x, 16) for x in re.findall(r"0x([0-9a-fA-F]+)U", body)], dtype=np.uint64).reshape(1024, 52)[:, :32]
+    rng = np.random.RandomState(5)
+    at = np.stack([rng.randint(0, 1024, 256), rng.randint(0, 32, 256)], axis=1)
+    out = {"sha256": hashlib.sha256(np.ascontiguousarray(nums, dtype="<u4").tobytes()).hexdigest(),
+           "entries": [[int(d), int(b), int(nums[d, b])] for d, b in at]}
+    json.dump(out, open(os.path.join(HERE, "sobol_reference.json"), "w"))
+
+
+def _cluster_mesh(verts, tris, cells):
+    """Vertex-clustering decimation: one vertex per occupied cell of a `cells`^3 grid over the bounding box (mean position,
+    uv and renormalised normal of the vertices it replaces); triangles that collapse or repeat are dropped."""
+    import numpy as np
+    from tungsten_b200 import scene as S
+    lo = verts["pos"].min(axis=0); ext = np.maximum(verts["pos"].max(axis=0) - lo, 1e-6)
+    c = np.minimum((((verts["pos"] - lo)/ext)*cells).astype(np.int64), cells - 1)
+    _, cell_of, counts = np.unique(c[:, 0]*cells*cells + c[:, 1]*cells + c[:, 2], return_inverse=True, return_counts=True)
+    out = np.zeros(len(counts), S.VERTEX_DTYPE)
+    for f in ("pos", "normal", "uv"):
+        acc = np.zeros((len(counts), out[f].shape[1]), np.float64)
+        np.add.at(acc, cell_of, verts[f].astype(np.float64))
+        out[f] = acc/counts[:, None]
+    out["normal"] /= np.maximum(np.linalg.norm(out["normal"], axis=1, keepdims=True), 1e-12)
+    idx = cell_of[np.stack([tris["v0"], tris["v1"], tris["v2"]], axis=1).astype(np.int64)]
+    keep = (idx[:, 0] != idx[:, 1]) & (idx[:, 1] != idx[:, 2]) & (idx[:, 0] != idx[:, 2])
+    _, first = np.unique(np.sort(idx[keep], axis=1), axis=0, return_index=True)
+    sel = np.where(keep)[0][np.sort(first)]
+    t = np.zeros(len(sel), S.TRI_DTYPE)
+    t["v0"], t["v1"], t["v2"] = idx[sel, 0], idx[sel, 1], idx[sel, 2]
+    t["material"] = tris["material"][sel]
+    return out, t
+
+
+def make_shipped_scenes():
+    """Shrunk copies of two scenes the reference ships, with the reference binary's renders of them (np.savez_compressed,
+    key "img"): tests/test_oracle_golden.py compares the oracle with these.
+      materialtest/   data/materialtest: the three meshes decimated by vertex clustering, envmap.hdr box-filtered to 64x32;
+                      ref_pathseed.npz = 64x64, 8 spp
+      hair_shipped/   data/example-scenes/hair: scene.json as shipped, curl.fiber reduced to 100 of its 10,000 strands (seed 7);
+                      ref_pathseed_lights.npz = its curves under an environment sphere + quad light, min_bounces 0;
+                      ref_pathseed_lights_nocurves.npz = the same lights without the curves (tells the strands' pixels apart);
+                      ref_pathseed.npz = the scene with its own emitters (skydome image: hair_sky/scene_sky_top.pfm, the same dome)
+                      all 90x300, 2 spp"""
+    import numpy as np
+    from tungsten_b200 import scene as S, synth
+
+    def render(d, js, name):
+        out = tempfile.mkdtemp()
+        p = os.path.join(d, "_render.json"); json.dump(js, open(p, "w"))
+        subprocess.check_call([os.path.join(ROOT, "oracle", "_ref", "tungsten_pathseed"), "-t", "8", "-d", out, p], stdout=subprocess.DEVNULL)
+        np.savez_compressed(os.path.join(d, name), img=S.load_pfm(os.path.join(out, "out.pfm")))
+        os.remove(p); shutil.rmtree(out)
+
+    src = os.path.join(REF, "data", "materialtest")
+    d = os.path.join(HERE, "materialtest"); os.makedirs(d, exist_ok=True)
+    js = json.load(open(os.path.join(src, "materialtest.json")))
+    for p in js["primitives"]:
+        if p["type"] == "mesh":
+            v, t = _cluster_mesh(*S.load_wo3(os.path.join(src, p["file"])), cells=12)
+            S.save_wo3(os.path.join(d, p["file"]), v, t)
+    env = S.load_rgbe(os.path.join(src, "envmap.hdr"))
+    fy, fx = env.shape[0]//32, env.shape[1]//64
+    synth.save_rgbe(os.path.join(d, "envmap.hdr"), env[:32*fy, :64*fx].reshape(32, fy, 64, fx, 3).mean(axis=(1, 3)).astype(np.float32))
+    js["camera"]["resolution"] = [64, 64]
+    js["renderer"].update(spp=8, spp_step=8, adaptive_sampling=False, stratified_sampler=True, hdr_output_file="out.pfm",
+                          output_file="out.png", overwrite_output_files=True)
+    json.dump(js, open(os.path.join(d, "scene.json"), "w"), indent=1)
+    render(d, js, "ref_pathseed.npz")
+
+    src = os.path.join(REF, "data", "example-scenes", "hair")
+    d = os.path.join(HERE, "hair_shipped"); os.makedirs(d, exist_ok=True)
+    shutil.copyfile(os.path.join(src, "scene.json"), os.path.join(d, "scene.json"))
+    ends, nodes = S.load_fiber(os.path.join(src, "curl.fiber"))
+    starts = np.concatenate([[0], ends[:-1]])
+    keep = np.sort(np.random.RandomState(7).choice(len(ends), 100, replace=False))
+    strands = [nodes[starts[k]:ends[k]] for k in keep]
+    S.save_fiber(os.path.join(d, "curl.fiber"), np.cumsum([len(s) for s in strands]).astype(np.uint32), np.concatenate(strands))
+    js = json.load(open(os.path.join(d, "scene.json")))
+    js["primitives"] = [p for p in js["primitives"] if p["type"] == "curves"] + [
+        {"name": "env", "type": "infinite_sphere", "emission": [0.5, 0.6, 0.8], "sample": True},
+        {"name": "key", "type": "quad", "emission": [60, 55, 50], "bsdf": {"type": "null"},
+         "transform": {"position": [3.0, 9.0, 6.0], "scale": [3, 1, 3], "rotation": [0, 0, 140]}}]
+    js["integrator"]["min_bounces"] = 0
+    for shipped_lights in (False, True):
+        if shipped_lights:
+            js = json.load(open(os.path.join(d, "scene.json")))
+        js["camera"]["resolution"] = [90, 300]
+        js["renderer"].update(spp=2, spp_step=2, adaptive_sampling=False, stratified_sampler=True, hdr_output_file="out.pfm",
+                              output_file="out.png", overwrite_output_files=True)
+        render(d, js, "ref_pathseed.npz" if shipped_lights else "ref_pathseed_lights.npz")
+        if not shipped_lights:
+            render(d, dict(js, primitives=[p for p in js["primitives"] if p["type"] != "curves"]), "ref_pathseed_lights_nocurves.npz")
+
+
 if __name__ == "__main__":
     make_kat()
+    make_sobol_reference()
     make_kat_curves()
     make_kat_bsdfs()
     make_kat_lights()
     make_kat_instances()
     make_kat_scene_hits()
     make_scenes()
+    make_shipped_scenes()

@@ -174,7 +174,7 @@ def test_multi_device_context_equals_single_device(scenes):
     for an adaptive step (block records merged from the GPU that owns each tile)."""
     import torch
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs two GPUs (gpurun --gpus 2)")
+        pytest.skip("needs two GPUs")
     fs = scenes("c1")
     one = lib.Context(fs, device=0)
     a, ca = one.render_tiles(4)

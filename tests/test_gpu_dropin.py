@@ -1,5 +1,5 @@
 """The literal drop-in: the reference renderer's own binary with `B200PathTraceIntegrator` linked in
-(integration/_build/tungsten_b200, built by `make -C oracle/ref dropin` where /root/reference is mounted) renders
+(oracle/_ref/dropin/tungsten_b200, built by `make -C oracle/ref dropin` where the reference's sources are at hand) renders
 scenes whose integrator type is "b200_path_tracer" on the GPU; its PFM output is compared with the framebuffers the
 reference's CPU integrator produced for the same scenes (tests/golden/*/ref_pathseed.pfm)."""
 import json
@@ -13,11 +13,11 @@ from tungsten_b200 import scene
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-EXE = os.path.join(ROOT, "integration", "_build", "tungsten_b200")
+EXE = os.path.join(ROOT, "oracle", "_ref", "dropin", "tungsten_b200")
 G = os.path.join(ROOT, "tests", "golden")
 
 
-@pytest.mark.skipif(not os.path.exists(EXE), reason="drop-in binary not built (needs /root/reference at build time)")
+@pytest.mark.skipif(not os.path.exists(EXE), reason="drop-in binary not built (needs the reference's sources at build time)")
 @pytest.mark.parametrize("name", ["cornell", "materials", "coat_env", "hair", "curves_plastic", "hair_sky", "dirac", "many_lights", "cube_city", "coats"])
 def test_reference_binary_with_b200_integrator(name, tmp_path):
     src = os.path.join(G, name)
@@ -50,7 +50,7 @@ def _run_dropin(tmp_path, js, name="b200.json", expect=None):
     return scene.load_pfm(str(tmp_path/"out"/"out.pfm")), out.stdout
 
 
-@pytest.mark.skipif(not os.path.exists(EXE), reason="drop-in binary not built (needs /root/reference at build time)")
+@pytest.mark.skipif(not os.path.exists(EXE), reason="drop-in binary not built (needs the reference's sources at build time)")
 def test_dropin_adaptive_sampling_as_shipped_scenes_use_it(tmp_path):
     """renderer.adaptive_sampling = true (the as-shipped setting of data/materialtest and the example scenes) through the
     literal drop-in: generateWork + per-block records in the adapter, tgb200_render_adaptive underneath, vs the reference
@@ -67,7 +67,7 @@ def test_dropin_adaptive_sampling_as_shipped_scenes_use_it(tmp_path):
     assert close >= 0.97
 
 
-@pytest.mark.skipif(not os.path.exists(EXE), reason="drop-in binary not built (needs /root/reference at build time)")
+@pytest.mark.skipif(not os.path.exists(EXE), reason="drop-in binary not built (needs the reference's sources at build time)")
 def test_dropin_writes_resume_state(tmp_path):
     """Integrator::saveRenderResumeData (Integrator.cpp:108-129) with the adapter's saveState: the resume file the drop-in
     writes after 16 spp holds the colour buffer and, behind it, the 4x4-block SampleRecords + the integrator's sampler state --
@@ -106,7 +106,7 @@ def test_dropin_writes_resume_state(tmp_path):
     assert sampler_state == st["sampler_state"]
 
 
-@pytest.mark.skipif(not os.path.exists(EXE), reason="drop-in binary not built (needs /root/reference at build time)")
+@pytest.mark.skipif(not os.path.exists(EXE), reason="drop-in binary not built (needs the reference's sources at build time)")
 def test_dropin_on_two_gpus_equals_one_gpu(tmp_path):
     """"devices": [0, 1] in the integrator block -> tgb_settings::devices: the library replicates the scene, deals the tiles
     in Morton order, gathers the shares on devices[0] over NVLink.  Under the per-path reseed contract the image does not

@@ -83,9 +83,10 @@ def test_coat_checker_envmap(scratch):
     _compare(fs, 8, frac_ok=0.9999, rel_rmse=1e-5, same_ray_count=False)     # measured: 1.00000, 1.2e-7
 
 
-def test_golden_scenes_against_reference_fixtures():
+def test_golden_scenes_against_reference_fixtures(tmp_path):
     """CUDA path vs the framebuffers rendered by the reference binary itself (tests/golden/*/ref_pathseed.pfm)."""
     import os
+    from test_oracle_golden import golden_scene_json
     g = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
     # the bit-exact fraction is informational (CUDA's sinf/cosf/expf differ from glibc's in the last ulp); the bar is "close"
     # curve scenes: see test_curves_and_hair for why their "close" bar is lower
@@ -96,7 +97,7 @@ def test_golden_scenes_against_reference_fixtures():
                                        ("cube_city", 0.3, 0.985),        # 151 analytic primitives: kept in BVH leaves (8 diffuse bounces: libm ulps add up)
                                        ("hair", 0.3, 0.97), ("hair_dark", 0.3, 0.97), ("hair_sky", 0.3, 0.97), ("curves_lambert", 0.5, 0.97),
                                        ("curves_plastic", 0.5, 0.97)]:
-        fs = scene.load_scene(os.path.join(g, name, "scene.json"))
+        fs = scene.load_scene(golden_scene_json(name, tmp_path))
         want = scene.load_pfm(os.path.join(g, name, "ref_pathseed.pfm"))
         ctx = lib.Context(fs); img, cnt = ctx.render_tiles(fs.spp); ctx.close()
         d = np.abs(img - want).max(axis=2)
